@@ -69,6 +69,9 @@ def parse():
     ap.add_argument("--row-graph", type=int, default=1, help="capture the row-sharded step in a CUDA graph (multicast exchange only)")
     ap.add_argument("--graph-comm", action="store_true",
                     help="EXPERIMENTAL (hung in round 1): capture the DP all-reduce + AdamW inside the CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (losses, gradients, updated parameters; rank 0) "
+                         "as DIR/<name>.npy in float32, for comparing two builds on the same seeded inputs")
     return ap.parse_args()
 
 
@@ -704,11 +707,32 @@ def row_shard_report(name, a, rank, world, dev):
     return out
 
 
+DUMP_BYTES = 60 * 2 ** 20
+
+
+def dump_outputs(out_dir, arrays, seed):
+    """Writes every tensor of `arrays` (name -> tensor) as float32 `out_dir/<name>.npy`, DUMP_BYTES of data in all.  The
+    smallest are written first and whole; a tensor larger than an even share of the bytes left keeps a seeded random
+    sample of its rows, in ascending row order, so that runs with the same arguments write the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    g = torch.Generator().manual_seed(seed)
+    left, todo = DUMP_BYTES, sorted(arrays.items(), key=lambda kv: (kv[1].numel(), kv[0]))
+    for i, (name, t) in enumerate(todo):
+        t = t.detach().float().cpu()
+        share = left // (len(todo) - i)
+        if 4 * t.numel() > share:
+            keep = share * t.shape[0] // (4 * t.numel())
+            t = t[torch.randperm(t.shape[0], generator=g)[:keep].sort().values]
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+        left -= 4 * t.numel()
+
+
 # ----------------------------------------------------------------------------------------------
 def main():
     global BATCH
     a = parse()
     BATCH = a.batch
+    torch.manual_seed(a.seed)         # dropout masks: the same arguments draw the same masks
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -723,11 +747,8 @@ def main():
     if a.impl == "reference":
         if rank != 0:
             return
-        # bounded sample: a CPU hot step of this workload takes ~0.4 s at the best thread count; cap the run at ~1 minute
-        executed = max(1, min(a.steps, 100))
-        cb = cpu_baseline(a.config, a.seed, executed, BATCH, a.cpu_threads)
-        cb["sample"] += f" ({executed} of the requested {a.steps} steps executed: bounded sample)"
-        line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": a.gpus, "steps": executed,
+        cb = cpu_baseline(a.config, a.seed, a.steps, BATCH, a.cpu_threads)
+        line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps,
                 "warmup": 1, "ms_per_step": round(cb["s_per_step"] * 1e3, 3), "higher_is_better": True, "scaling": "weak",
                 "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": config, "cpu_baseline": cb,
                 "e2e": {"value": cb["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
@@ -737,8 +758,8 @@ def main():
     if a.impl == "stock-gpu":
         if rank != 0:
             return
-        sg = stock_gpu_baseline(a.config, a.seed, min(a.steps, 200), max(a.warmup, 3), BATCH, os.environ.get("MMSSL_STOCK_DEVICE", "cuda:0"))
-        print(json.dumps({"impl": "stock-torch-gpu", "metric": METRIC, "value": sg["value"], "unit": UNIT, "n_gpus": 1, "steps": min(a.steps, 200),
+        sg = stock_gpu_baseline(a.config, a.seed, a.steps, max(a.warmup, 3), BATCH, os.environ.get("MMSSL_STOCK_DEVICE", "cuda:0"))
+        print(json.dumps({"impl": "stock-torch-gpu", "metric": METRIC, "value": sg["value"], "unit": UNIT, "n_gpus": 1, "steps": a.steps,
                           "warmup": max(a.warmup, 3), "ms_per_step": sg["ms_per_step"], "higher_is_better": True, "dtype": "f32",
                           "data": "synthetic", "config": config, "comparator": sg}))
         return
@@ -804,6 +825,13 @@ def main():
     pts = [e0] + marks + [e1]
     seg_steps = [seg] * (n_seg - 1) + [a.steps - seg * (n_seg - 1)]
     seg_ms = [pts[i].elapsed_time(pts[i + 1]) / seg_steps[i] for i in range(n_seg)]
+    if a.dump_outputs:                # before (B) steps the parameters on
+        if rank == 0:
+            from mmssl_b200.engine import LIVE
+            hs = trainer.hs
+            dump_outputs(a.dump_outputs, {"losses": hs.out5, **{"grad." + k: hs.grads[k] for k in LIVE},
+                                          **{"param." + k: hs.P[k] for k in LIVE}}, a.seed)
+        barrier()
 
     # ---------------- (B) end to end through the public API (pinned host -> device, loss read back)
     for w in range(min(3, a.warmup)):

@@ -11,7 +11,6 @@ The patches are undone by ``monkeypatch``; nothing under mmssl_b200/ knows about
 import contextlib
 import ctypes as C
 import os
-import sys
 import weakref
 
 import torch
@@ -135,10 +134,9 @@ def emulated_device(monkeypatch, guard: bool = False):
         clear()
     monkeypatch.setattr(_lib, "load", lambda require_device=False: lib)
     monkeypatch.setattr(_lib, "_lib", lib)
-    null_stream = lambda: C.c_void_p(0)
-    for name, mod in list(sys.modules.items()):
-        if name.startswith("mmssl_b200") and mod is not None and hasattr(mod, "stream"):
-            monkeypatch.setattr(mod, "stream", null_stream)
+    # the NULL stream comes from the patched torch.cuda.current_stream, which _lib.stream() reads at every call.  Patching
+    # `stream` in the modules instead would leak: a module first imported during the test keeps the patched function it
+    # imported, and on a machine with a GPU its later launches would bypass the current stream (and any graph capture on it).
     monkeypatch.setattr(torch.Tensor, "cuda", lambda self, *a, **k: self.clone())   # a copy, like a real host->device transfer
     real_to = torch.Tensor.to
 
